@@ -45,7 +45,30 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-other-configs", action="store_true", help="skip the cfg3/cfg4/cfg5 table of the default cfg2 run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed pass returned (solutions, fitness, success, steps of every query) "
+                                                          "as DIR/<name>.npy in float64, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, slab, n_vars, B):
+    """The answers a caller of the timed path receives, from its [B][n_vars + 3] result slab (all ranks' queries in query order).
+    Above DUMP_MAX_BYTES only a fixed, seeded sample of the queries is written, their indices in query_index.npy."""
+    from bio_ik_b200.distributed import unpack_slab
+    os.makedirs(out_dir, exist_ok=True)
+    out = unpack_slab(slab, n_vars, B)
+    rows = DUMP_MAX_BYTES // ((n_vars + 4) * 8)
+    if B > rows:
+        idx = np.sort(np.random.default_rng(0).choice(B, rows, replace=False))
+        out = {k: v[idx] for k, v in out.items()}
+        out["query_index"] = idx
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -211,9 +234,9 @@ def fp64_peak(clocks):
         return 148 * 64 * 2 * mhz * 1e6 / 1e12, "fallback: nominal 148 SMs x 64 FP64 FMA lanes x 2 x sampled SM clock (profiles/fp64_peak.json absent)"
 
 
-def measure(args, config, B, steps, warmup, env, cpu_seconds, full):
+def measure(args, config, B, steps, warmup, env, cpu_seconds, full, dump_dir=None):
     """One bench measurement of `config` at B queries per GPU: device-resident value, host-buffer e2e, kernel timing, CPU arm.
-    env = dict(torch, dist, world, rank, local_rank, dev, stream)."""
+    env = dict(torch, dist, world, rank, local_rank, dev, stream).  dump_dir: where rank 0 writes the results of the last timed pass."""
     torch, dist, world, rank, dev, stream = env["torch"], env["dist"], env["world"], env["rank"], env["dev"], env["stream"]
     from bio_ik_b200 import workloads
     from bio_ik_b200.distributed import DeviceShardedSolver
@@ -264,6 +287,8 @@ def measure(args, config, B, steps, warmup, env, cpu_seconds, full):
     barrier()
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if sampler else None
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, sharded.gathered.cpu().numpy(), n_vars, world * B)
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     launches = solver.launch_count() - launches0
     ev_ms, ev_n, ser_ms, ser_n = solver.kernel_time(reset=True)
@@ -393,7 +418,7 @@ def main():
     torch.cuda.set_stream(stream)
     env = dict(torch=torch, dist=dist, world=world, rank=rank, local_rank=local_rank, dev=dev, stream=stream,
                flush=torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev))  # > 126 MB L2
-    m = measure(args, args.config, args.batch, args.steps, args.warmup, env, 0.0 if args.no_cpu_baseline else args.cpu_seconds, True)
+    m = measure(args, args.config, args.batch, args.steps, args.warmup, env, 0.0 if args.no_cpu_baseline else args.cpu_seconds, True, dump_dir=args.dump_outputs)
 
     # BASELINE.json's other configurations on the same box (N = 1 only): GPU value, e2e, the reference's CPU arm and the bound fraction
     others = None

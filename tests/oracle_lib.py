@@ -222,13 +222,18 @@ class Reference:
     def table(self, which, seed, n=1 << 23):
         return np.ctypeslib.as_array(self.lib.ref_table(which, seed), shape=(1 << 23,))[:n].copy()
 
+    def effective_link_origins(self, robot):
+        """[n_links][7]: the link origins as the reference stores them (its Isometry3d -> quaternion conversion, forward_kinematics.h:203)"""
+        out = np.zeros((len(robot.links), 7))
+        r = robot.to_abi()
+        self._check(self.lib.ref_effective_link_origins(C.byref(r), _abi.dptr(out)))
+        return out
+
     def effective_robot(self, robot):
         """copy of `robot` whose link origins are the frames the reference derives from the same robot (its
         Isometry3d -> quaternion conversion, forward_kinematics.h:203); differs from the input by at most an ulp"""
         import copy
-        out = np.zeros((len(robot.links), 7))
-        r = robot.to_abi()
-        self._check(self.lib.ref_effective_link_origins(C.byref(r), _abi.dptr(out)))
+        out = self.effective_link_origins(robot)
         src = robot.arrays["link_origin"].reshape(-1, 7)
         sign = np.where((out[:, 3:] * src[:, 3:]).sum(axis=1) < 0, -1.0, 1.0)[:, None]  # q and -q are the same rotation
         assert np.allclose(out[:, :3], src[:, :3], rtol=0, atol=0) and np.allclose(out[:, 3:] * sign, src[:, 3:], rtol=0, atol=1e-14)

@@ -1,11 +1,12 @@
 """SURVEY.md §8(b): the drop-in boundary, compiled.  adapter/ik_evolution_2_b200.cpp (the translation unit a bio_ik maintainer adds)
 is built INSIDE the reference's own solver framework - IKBase, IKFactory, Problem, the goal classes, IKParallel where they lie under
-/root/reference, third-party headers from oracle/shims (oracle/adapter_harness.cpp -> oracle/_ref/libbioik_adapter.so, prebuilt here,
-travels to the GPU box) - and driven through the reference's types:
+the reference's sources, third-party headers from oracle/shims (oracle/adapter_harness.cpp -> oracle/_ref/libbioik_adapter.so) - and
+driven through the reference's types:
     IKFactory::create("bio2_memetic_b200") -> initialize(problem) -> step() x k -> getSolution()      (src/ik_base.h:138-154)
     IKParallel(params).solve()                                                                     (src/ik_parallel.h:148-269)
 The GPU tests demand the same solution BITS as the C ABI called directly (bioik_begin / bioik_step / bioik_get_solution and
-bioik_solve_islands)."""
+bioik_solve_islands); they read the adapter's and the reference's answers from tests/golden/reference/ (tests/reference_store.py),
+recorded from that library on a B200, so only the test of the library itself needs the reference's sources."""
 import ctypes as C
 import os
 import subprocess
@@ -14,6 +15,7 @@ import numpy as np
 import pytest
 
 import oracle_lib
+import reference_store
 from bio_ik_b200 import _abi, goals as G, robots, workloads
 from bio_ik_b200.problem import Problem
 
@@ -26,7 +28,7 @@ def load_adapter():
         ge.build_cuda()
         subprocess.run(["make", "-C", oracle_lib.ORACLE_DIR, "-s", "adapter"], check=True)
     if not os.path.exists(ADAPTER_LIB):
-        pytest.skip("oracle/_ref/libbioik_adapter.so is not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libbioik_adapter.so is not built (it needs the reference's sources at build time)")
     lib = C.CDLL(ADAPTER_LIB)
     dp, ip = _abi.c_double_p, _abi.c_int32_p
     RP, PP = C.POINTER(_abi.BioikRobot), C.POINTER(_abi.BioikProblem)
@@ -73,6 +75,16 @@ def test_adapter_registers_with_the_reference_factory_and_has_no_cpu_fallback():
 
 
 # ---------------------------------------------------------------------------------------------- GPU
+ref = reference_store.reference_fixture("adapter")
+
+
+@pytest.fixture
+def adapter(request):
+    a = reference_store.StoredAdapter(reference_store.store_name("adapter", request), load_adapter)
+    yield a
+    a.close()
+
+
 def effective(ref, w, B):
     return ref.effective_robot(w.robot), ref.effective_goal_params(w.robot, w.problem, w.goal_params, B)
 
@@ -80,21 +92,16 @@ def effective(ref, w, B):
 @pytest.mark.gpu
 @pytest.mark.parametrize("solver,mode", [("bio2_memetic_b200", "bio2_memetic"), ("bio2_b200", "bio2"), ("bio2_memetic_l_b200", "bio2_memetic_l")])
 @pytest.mark.parametrize("use_clone", [0, 1])
-def test_factory_initialize_step_get_solution_equals_the_c_abi(oracle, solver, mode, use_clone, monkeypatch):
+def test_factory_initialize_step_get_solution_equals_the_c_abi(oracle, adapter, ref, solver, mode, use_clone, monkeypatch):
     """IKFactory::create -> initialize -> step() x k -> getSolution() through the reference's types (optionally on an
     IKFactory::clone copy, re-initialised for three queries in a row) returns the solution bits of bioik_begin / bioik_step /
     bioik_get_solution and of bioik_solve_islands called directly."""
     from bio_ik_b200.solver import IKSolver
-    lib = load_adapter()
-    ref = oracle_lib.Reference("strict")
     islands, steps, Q, random_seed = 16, 7, 3, 5
     monkeypatch.setenv("BIOIK_B200_ISLANDS", str(islands))
     w = workloads.make("cfg2", lambda rm, pr, v: oracle.fk(rm, pr, v), batch=Q)
     robot, gp = effective(ref, w, Q)
-    r, p = w.robot.to_abi(), w.problem.to_abi()
-    got = np.zeros((Q, w.robot.n_vars))
-    rc = lib.adapter_steps(C.byref(r), C.byref(p), solver.encode(), random_seed, Q, _abi.dptr(np.ascontiguousarray(w.goal_params)), _abi.dptr(np.ascontiguousarray(w.seeds)), steps, use_clone, _abi.dptr(got))
-    assert rc == 0, lib.ref_last_error().decode()
+    got = adapter.steps(w.robot, w.problem, solver, random_seed, w.goal_params, w.seeds, steps, use_clone)
     direct = IKSolver(robot, mode=mode, population=18, random_seed=random_seed, device=0).initialize(w.problem)
     rs = (random_seed + np.arange(islands)).astype(np.uint32)
     for q in range(Q):
@@ -110,27 +117,21 @@ def test_factory_initialize_step_get_solution_equals_the_c_abi(oracle, solver, m
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("threads", [1, 2])
-def test_ikparallel_drives_the_gpu_solver_unchanged(oracle, threads, monkeypatch):
+def test_ikparallel_drives_the_gpu_solver_unchanged(oracle, adapter, ref, threads, monkeypatch):
     """The reference's driver - IKParallel::solve with its thread pool, 4-step bursts, its own exact FK + checkSolution on what the
     solver returns (src/ik_parallel.h:148-269) - around the adapter.  It stops at the first burst after which the returned vector
     passes the reference's success test; the same loop written against the C ABI gives the same bits and the same burst count."""
     from bio_ik_b200.solver import IKSolver
-    lib = load_adapter()
-    ref = oracle_lib.Reference("strict")
     islands, random_seed, Q = 32, 3, 4
     monkeypatch.setenv("BIOIK_B200_ISLANDS", str(islands))
     w = workloads.make("cfg2", lambda rm, pr, v: oracle.fk(rm, pr, v), batch=Q)
     robot, gp = effective(ref, w, Q)
-    r, p = w.robot.to_abi(), w.problem.to_abi()
     direct = IKSolver(robot, mode="bio2_memetic", population=18, random_seed=random_seed, device=0).initialize(w.problem)
     solved = 0
     for q in range(Q):
-        sol, succ, fit, iters = np.zeros(w.robot.n_vars), C.c_int32(), C.c_double(), C.c_int32()
-        rc = lib.adapter_parallel(C.byref(r), C.byref(p), b"bio2_memetic_b200", random_seed, threads, _abi.dptr(np.ascontiguousarray(w.goal_params[q])), _abi.dptr(np.ascontiguousarray(w.seeds[q])), 20.0, _abi.dptr(sol),
-                                  C.byref(succ), C.byref(fit), C.byref(iters))
-        assert rc == 0, lib.ref_last_error().decode()
-        assert succ.value == 1  # reachable PR2-arm poses, 32+ islands: the reference's own test accepts the GPU's answer
-        solved += succ.value
+        sol, succ, fit, iters = adapter.parallel(w.robot, w.problem, "bio2_memetic_b200", random_seed, threads, w.goal_params[q], w.seeds[q], 20.0)
+        assert succ == 1  # reachable PR2-arm poses, 32+ islands: the reference's own test accepts the GPU's answer
+        solved += succ
         # the reference's exact FK of the returned vector really is at the goal
         tip = oracle.fk(w.robot, w.problem, sol[None])[0, 0]
         assert np.abs(tip[:3] - w.goal_params[q, 0, :3]).max() < 1e-4
@@ -144,7 +145,7 @@ def test_ikparallel_drives_the_gpu_solver_unchanged(oracle, threads, monkeypatch
                 a = direct.get_solution(wrap=False)
                 if a["success"][0] or bursts > 200:
                     break
-            assert bursts == iters.value and np.array_equal(sol, a["solutions"][0]), (q, bursts, iters.value)
+            assert bursts == iters and np.array_equal(sol, a["solutions"][0]), (q, bursts, iters)
     assert solved == Q
 
 
@@ -174,13 +175,11 @@ def test_resumable_steps_cost_no_restart(oracle):
 
 
 @pytest.mark.gpu
-def test_adapter_flattens_a_balance_goal_from_the_urdf_inertials(oracle, monkeypatch):
+def test_adapter_flattens_a_balance_goal_from_the_urdf_inertials(oracle, adapter, ref, monkeypatch):
     """BalanceGoal through the reference's types: the adapter reads the link inertials from RobotModel::getURDF() like
     BalanceGoal::describe does, the reference's Problem::initialize makes every link with mass a tip link, and the device answer equals
     the C ABI called with the same flattened problem."""
     from bio_ik_b200.solver import IKSolver
-    lib = load_adapter()
-    ref = oracle_lib.Reference("strict")
     islands, steps, random_seed = 8, 5, 2
     monkeypatch.setenv("BIOIK_B200_ISLANDS", str(islands))
     rm, groups = robots.balancing_tree()
@@ -189,10 +188,7 @@ def test_adapter_flattens_a_balance_goal_from_the_urdf_inertials(oracle, monkeyp
     rng = np.random.default_rng(4)
     seeds = workloads.sample_configurations(rm, pr.active_variables, 1, rng)
     gp = pr.default_goal_params()[None]
-    r, p = rm.to_abi(), pr.to_abi()
-    got = np.zeros((1, rm.n_vars))
-    rc = lib.adapter_steps(C.byref(r), C.byref(p), b"bio2_memetic_b200", random_seed, 1, _abi.dptr(np.ascontiguousarray(gp)), _abi.dptr(np.ascontiguousarray(seeds)), steps, 0, _abi.dptr(got))
-    assert rc == 0, lib.ref_last_error().decode()
+    got = adapter.steps(rm, pr, "bio2_memetic_b200", random_seed, gp, seeds, steps, 0)
     direct = IKSolver(ref.effective_robot(rm), mode="bio2_memetic", population=18, random_seed=random_seed, device=0).initialize(pr)
     rs = (random_seed + np.arange(islands)).astype(np.uint32)
     want = direct.solve_islands(ref.effective_goal_params(rm, pr, gp, 1), seeds, islands, steps, rng_seeds=rs, early_exit=2, wrap=False)

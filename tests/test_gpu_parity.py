@@ -9,11 +9,13 @@ import pytest
 
 import gpu_util
 import oracle_lib
+import reference_store
 from bio_ik_b200 import _abi, goals as G, robots, workloads
 from bio_ik_b200.problem import Problem
 from bio_ik_b200.solver import BioIKError, IKSolver
 
 pytestmark = pytest.mark.gpu
+ref = reference_store.reference_fixture("gpu_parity")
 
 
 def ofk(oracle):
@@ -388,18 +390,14 @@ def test_solve_islands_default_goal_parameters_and_seeds(oracle):
 
 
 # ---------------------------------------------------------------------------------------------
-# the CUDA path against the REFERENCE'S OWN CODE (oracle/_ref, prebuilt where /root/reference exists; travels to the GPU box)
+# the CUDA path against the REFERENCE'S OWN CODE (its answers stored under tests/golden/reference/, see tests/reference_store.py)
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("name,B,pop,steps", [("cfg2", 256, 128, 25), ("cfg2", 64, 18, 25), ("cfg1", 1, 64, 25), ("cfg4", 16, 128, 10)])
-def test_gpu_equals_the_reference_code_with_contract_math(name, B, pop, steps):
+def test_gpu_equals_the_reference_code_with_contract_math(ref, name, B, pop, steps):
     """No oracle in between: the reference's src/ik_evolution_2.cpp + src/problem.cpp + forward_kinematics.h, compiled in place
     (oracle/ref_harness.cpp), with its two libm calls sin / cos swapped for the arithmetic contract's det_sincos and its child pool
     re-sized to `pop` - against bioik_solve_batch on the GPU.  Bit-identical joint angles, fitness, success flags and every
     species' genes and gradients (single-tip problems: quirk Q2 does not apply)."""
-    try:
-        ref = oracle_lib.Reference("strict")
-    except (FileNotFoundError, OSError) as e:
-        pytest.skip(f"reference build not available here: {e}")
     w = workloads.make(name, lambda rm, pr, v: oracle_lib.Oracle().fk(rm, pr, v), batch=B)
     B = len(w.rng_seeds)
     # the numbers the reference stores after its own normalising constructors / Isometry3d conversion (ulp-level changes)
@@ -413,37 +411,30 @@ def test_gpu_equals_the_reference_code_with_contract_math(name, B, pop, steps):
     finally:
         ref.contract_math(False)
     for k in ("genes", "gradients", "species_fitness", "solutions", "fitness"):
-        assert np.array_equal(got[k], want[k]), k
-    assert np.array_equal(res["success"], want["success"]) and np.array_equal(res["solutions"], want["solutions"])
+        assert reference_store.same(got[k], want[k]), k
+    assert reference_store.same(res["success"], want["success"]) and reference_store.same(res["solutions"], want["solutions"])
 
 
 @pytest.mark.parametrize("name,B,pop,steps", [("cfg3", 64, 128, 25), ("cfg5", 48, 128, 12), ("cfg3", 32, 18, 25)])
-def test_gpu_reference_stale_tip_mode_equals_the_reference_code(oracle, name, B, pop, steps):
+def test_gpu_reference_stale_tip_mode_equals_the_reference_code(oracle, ref, name, B, pop, steps):
     """Multi-tip problems in the reference-quirk mode (BIOIK_OPT_REFERENCE_STALE_TIPS): bit-identical to the oracle's emulation
-    of quirk Q2 and - where oracle/_ref is present - to the reference's own code (contract sin / cos, phenotypes3 pre-filled
-    with identity frames by the harness), i.e. all five BASELINE configurations match the reference's code on the GPU."""
+    of quirk Q2 and to the reference's own code (contract sin / cos, phenotypes3 pre-filled with identity frames by the
+    harness), i.e. all five BASELINE configurations match the reference's code on the GPU."""
     w = workloads.make(name, ofk(oracle), batch=B)
     cfg = oracle_lib.make_cfg(population=pop)
-    robot, gp = w.robot, w.goal_params
-    ref = None
-    try:
-        ref = oracle_lib.Reference("strict")
-        robot, gp = ref.effective_robot(w.robot), ref.effective_goal_params(w.robot, w.problem, w.goal_params, B)
-    except (FileNotFoundError, OSError):
-        pass
+    robot, gp = ref.effective_robot(w.robot), ref.effective_goal_params(w.robot, w.problem, w.goal_params, B)
     solver = IKSolver(robot, mode="bio2_memetic", population=pop, random_seed=1, device=0, reference_stale_tips=True).initialize(w.problem)
     got = solver.trace(gp, w.seeds, w.rng_seeds, steps)
     want = oracle.solve(robot, w.problem, cfg, gp, w.seeds, w.rng_seeds, steps, flags=8)
     for k in ("genes", "gradients", "species_fitness", "solutions", "fitness"):
         assert np.array_equal(got[k], want[k]), k
-    if ref is not None:
-        ref.contract_math(True)
-        try:
-            r = ref.solve(w.robot, w.problem, cfg, w.goal_params, w.seeds, w.rng_seeds, steps)
-        finally:
-            ref.contract_math(False)
-        for k in ("genes", "gradients", "species_fitness", "solutions", "fitness"):
-            assert np.array_equal(got[k], r[k]), ("reference", k)
+    ref.contract_math(True)
+    try:
+        r = ref.solve(w.robot, w.problem, cfg, w.goal_params, w.seeds, w.rng_seeds, steps)
+    finally:
+        ref.contract_math(False)
+    for k in ("genes", "gradients", "species_fitness", "solutions", "fitness"):
+        assert reference_store.same(got[k], r[k]), ("reference", k)
     # and the default mode differs on these problems (documented deviation Q2)
     plain = IKSolver(robot, mode="bio2_memetic", population=pop, random_seed=1, device=0).initialize(w.problem).trace(gp, w.seeds, w.rng_seeds, steps)
     assert not np.array_equal(plain["genes"], got["genes"])
@@ -465,10 +456,10 @@ def floating_problem(oracle, group, B, seed=1, maker=None):
 
 @pytest.mark.parametrize("maker", [robots.floating_base_arm, robots.planar_base_arm])
 @pytest.mark.parametrize("group,mode,gens", [("whole_arm", "q", 8), ("all", "q", 8), ("all", 0, 16), ("whole_arm", "l", 8)])
-def test_floating_and_planar_base_joints(oracle, group, mode, gens, maker):
+def test_floating_and_planar_base_joints(oracle, ref, group, mode, gens, maker):
     """SURVEY.md §8(f) row 4: a FLOATING joint on the chain (src/forward_kinematics.h:120-127 joint frame, :695-726 numeric
     Jacobian through frameTwist, src/ik_evolution_2.cpp:118-126,320-324 quaternion-gene normalisation) - bit-identical to the
-    oracle and, where oracle/_ref is present, to the reference's own code (contract sin / cos / acos; quirk mode for the
+    oracle and to the reference's own code (contract sin / cos / acos; quirk mode for the
     two-tip problem, where the base moves both tips but the arm joints only one).  PLANAR joints take the same numeric route;
     their joint frame is MoveIt's computeTransform + Eigen's matrix -> quaternion, restated (oracle/shims/README.md)."""
     B, pop, steps = 48, 64 if maker is robots.floating_base_arm else 128, 12
@@ -480,10 +471,6 @@ def test_floating_and_planar_base_joints(oracle, group, mode, gens, maker):
     want = oracle.solve(rm, pr, cfg, gp, seeds, rs, steps)
     for k in ("genes", "gradients", "species_fitness", "solutions", "fitness"):
         assert np.array_equal(got[k], want[k]), k
-    try:
-        ref = oracle_lib.Reference("strict")
-    except (FileNotFoundError, OSError):
-        return
     robot, gpe = ref.effective_robot(rm), ref.effective_goal_params(rm, pr, gp, B)
     got = IKSolver(robot, mode=name, population=pop, random_seed=1, device=0, reference_stale_tips=True).initialize(pr).trace(gpe, seeds, rs, steps)
     ref.contract_math(True)
@@ -492,7 +479,7 @@ def test_floating_and_planar_base_joints(oracle, group, mode, gens, maker):
     finally:
         ref.contract_math(False)
     for k in ("genes", "gradients", "species_fitness", "solutions", "fitness"):
-        assert np.array_equal(got[k], r[k]), ("reference", k)
+        assert reference_store.same(got[k], r[k]), ("reference", k)
 
 
 def test_cancel_from_another_thread(oracle):
@@ -551,7 +538,7 @@ def test_balance_goal_on_gpu(oracle, first):
 
 
 @pytest.mark.parametrize("name,B", [("cfg2", 512), ("cfg3", 128), ("cfg5", 64)])
-def test_gpu_against_the_reference_as_shipped(oracle, name, B):
+def test_gpu_against_the_reference_as_shipped(oracle, ref, name, B):
     """The GPU against the reference's own code with NOTHING swapped (libm sin / cos, oracle/_ref/libbioik_ref_strict.so), in the
     tolerance BASELINE.json names:
       * per-component quantities - exact FK tip frames, delta frames, approximate fitness - agree to 1e-12 (measured <= 3e-15: the
@@ -560,18 +547,23 @@ def test_gpu_against_the_reference_as_shipped(oracle, name, B):
         differences, and the reference's own IEEE and -ffast-math builds already disagree after ONE step on 997 of 1000 queries
         (profiles/tolerance_study.py -> profiles/r02_tolerance_study.json).  What is comparable is the distribution: success rate
         within sampling error and the same median fitness scale after 25 steps."""
-    try:
-        ref = oracle_lib.Reference("strict")
-    except (FileNotFoundError, OSError) as e:
-        pytest.skip(f"reference build not available here: {e}")
     w = workloads.make(name, ofk(oracle), batch=B)
+    ref.keep_values("success", "fitness")  # compared as a distribution
     robot, gp = ref.effective_robot(w.robot), ref.effective_goal_params(w.robot, w.problem, w.goal_params, B)
     solver = IKSolver(robot, mode="bio2_memetic", population=128, random_seed=1, device=0).initialize(w.problem)
     rng = np.random.default_rng(0)
     n = len(w.problem.active_variables)
     base = workloads.sample_configurations(w.robot, w.problem.active_variables, B, rng)
     genes = base[:, w.problem.active_variables][:, None, :] + rng.normal(0, 0.05, (B, 8, n))
-    r = ref.approx_fitness(w.robot, w.problem, w.goal_params, w.seeds, base, genes)  # libm: the reference exactly as it is
+    stored = ref.approx_fitness(w.robot, w.problem, w.goal_params, w.seeds, base, genes)  # libm: the reference exactly as it is
+    # its numbers: the oracle with libm sin / cos on the reference's link frames reproduces them bit for bit (checked against the stored digests)
+    oracle.component_flags(1)
+    try:
+        r = dict(tips=oracle.fk(robot, w.problem, base, libm=True), delta=oracle.approx(robot, w.problem, base)[0], primary=oracle.approx_fitness(robot, w.problem, gp, w.seeds, base, genes)[0])
+    finally:
+        oracle.component_flags(0)
+    for k in ("tips", "delta", "primary"):
+        assert reference_store.same(r[k], stored[k]), k
     assert np.allclose(solver.fk(base), r["tips"], rtol=1e-12, atol=1e-12)
     assert np.allclose(solver.approx(base), np.where(np.abs(r["delta"]) > 0, r["delta"], solver.approx(base)), rtol=1e-10, atol=1e-12)
     prim, _ = solver.approx_fitness(gp, w.seeds, base, genes)

@@ -7,13 +7,14 @@ Every comparison below is BIT-EXACT.  The oracle runs with one switch flipped: l
 calls, forward_kinematics.h:95-109) instead of the arithmetic contract's det_sincos, which is the single
 documented numeric deviation of the product path (DESIGN.md §3, <= 2 ulp, tested in test_oracle.py).
 
-The library is built by `make -C oracle ref` (done by __graft_entry__.build()) wherever /root/reference exists;
-where neither the sources nor a prebuilt oracle/_ref/ are present these tests skip.
+The reference's answers come from tests/golden/reference/ (tests/reference_store.py), recorded from that library, which is
+built by `make -C oracle ref` (done by __graft_entry__.build()) where the reference's sources are available.
 """
 import numpy as np
 import pytest
 
 import oracle_lib
+import reference_store
 from bio_ik_b200 import goals as G, robots, workloads
 from bio_ik_b200.problem import Problem
 
@@ -23,12 +24,7 @@ KEYS = ("solutions", "fitness", "success", "steps", "genes", "gradients", "speci
 MODES = {"bio2": (0, 16), "bio2_memetic": ("q", 8), "bio2_memetic_l": ("l", 8)}
 
 
-@pytest.fixture(scope="module")
-def ref():
-    try:
-        return oracle_lib.Reference("strict")
-    except (FileNotFoundError, OSError) as e:
-        pytest.skip(f"reference build not available here: {e}")
+ref = reference_store.reference_fixture("reference_pin")
 
 
 @pytest.fixture(scope="module")
@@ -46,7 +42,7 @@ def compare(oracle, ref, rm, pr, cfg, gp, seeds, rs, steps, early_exit=False):
     a = oracle.solve(ref.effective_robot(rm), pr, cfg, gpe, seeds, rs, steps, early_exit=early_exit, flags=LIBM | STALE)
     b = ref.solve(rm, pr, cfg, gp, seeds, rs, steps, early_exit=early_exit)
     for k in KEYS:
-        assert np.array_equal(a[k], b[k]), (k, int((a[k].reshape(B, -1) != b[k].reshape(B, -1)).any(axis=1).sum()), "of", B)
+        assert reference_store.same(a[k], b[k]), k
     return a
 
 
@@ -54,8 +50,8 @@ def test_lookup_tables_are_the_references(ref, oracle):
     """Random::Random (utils.h) fills both 2^23 tables from the seed; the oracle's Tables (and through it the product's make_tables) match it."""
     for seed in (1, 7):
         u, g = oracle.table_arrays(seed)
-        assert np.array_equal(ref.table(0, seed), u)
-        assert np.array_equal(ref.table(1, seed), g)
+        assert reference_store.same(u, ref.table(0, seed))
+        assert reference_store.same(g, ref.table(1, seed))
 
 
 @pytest.mark.parametrize("mode", list(MODES))
@@ -98,7 +94,7 @@ def test_other_configs(ref, oracle, name, B, steps):
         compare(oracle, ref, w.robot, w.problem, cfg, w.goal_params, w.seeds, w.rng_seeds, steps)
 
 
-def test_stale_tip_quirk_is_confined_to_multi_tip_problems(ref, oracle):
+def test_stale_tip_quirk_is_confined_to_multi_tip_problems(oracle):
     """Quirk Q2: the reference's computeApproximateMutation1 (forward_kinematics.h:940) skips the tips a variable does
     not move, so the memetic gradient probe (ik_evolution_2.cpp:469-470) scores those tips on stale frames left by an
     earlier call (uninitialised heap memory the first time; the harness pre-fills the buffer to make runs reproducible).
@@ -144,17 +140,18 @@ def test_goal_classes_and_problem_initialize(ref, oracle):
     gp = np.repeat(pr.default_goal_params()[None], B, 0)
     gp[:, 0, 0:3] += rng.normal(0, 0.1, (B, 3))
     gpe = ref.effective_goal_params(rm, pr, gp, B)
+    ref.keep_values("delta")  # compared where the variable moves the tip
     b = ref.approx_fitness(rm, pr, gp, seeds, base, genes)
     oracle.component_flags(LIBM)
     try:
-        assert np.array_equal(oracle.fk(rm, pr, base, libm=True), b["tips"])
+        assert reference_store.same(oracle.fk(rm, pr, base, libm=True), b["tips"])
         delta, mask = oracle.approx(rm, pr, base)
         assert np.array_equal(delta[mask != 0], b["delta"][mask != 0])
-        assert np.array_equal(oracle.approx_frames(rm, pr, base, genes), b["frames"])
+        assert reference_store.same(oracle.approx_frames(rm, pr, base, genes), b["frames"])
         prim, sec = oracle.approx_fitness(rm, pr, gpe, seeds, base, genes)
     finally:
         oracle.component_flags(0)
-    assert np.array_equal(prim, b["primary"]) and np.array_equal(sec, b["secondary"])
+    assert reference_store.same(prim, b["primary"]) and reference_store.same(sec, b["secondary"])
     assert np.abs(sec).min() > 0  # the secondary goals really contribute
     # ...and the same problem through whole solver steps
     cfg = oracle_lib.make_cfg(population=18)
@@ -175,6 +172,7 @@ def test_cone_goal_is_the_one_exception(ref, oracle):
     base = workloads.sample_configurations(rm, pr.active_variables, B, rng)
     genes = base[:, pr.active_variables][:, None, :] + rng.normal(0, 0.2, (B, M, n))
     gp = np.repeat(pr.default_goal_params()[None], B, 0)
+    ref.keep_values("primary")
     b = ref.approx_fitness(rm, pr, gp, base, base, genes)
     oracle.component_flags(LIBM)
     try:
@@ -198,7 +196,7 @@ def test_reference_with_contract_math_equals_the_default_oracle(ref, oracle):
             a = oracle.solve(ref.effective_robot(w.robot), w.problem, cfg, gpe, w.seeds, w.rng_seeds, 25)  # default flags: the arithmetic contract
             b = ref.solve(w.robot, w.problem, cfg, w.goal_params, w.seeds, w.rng_seeds, 25)
             for k in KEYS:
-                assert np.array_equal(a[k], b[k]), (name, k)
+                assert reference_store.same(a[k], b[k]), (name, k)
         # ConeGoal, now to the bit
         rm, groups = robots.pr2_like()
         g = groups["all"]
@@ -211,7 +209,7 @@ def test_reference_with_contract_math_equals_the_default_oracle(ref, oracle):
         gp = np.repeat(pr.default_goal_params()[None], B, 0)
         b = ref.approx_fitness(rm, pr, gp, base, base, genes)
         prim, _ = oracle.approx_fitness(ref.effective_robot(rm), pr, ref.effective_goal_params(rm, pr, gp, B), base, base, genes)
-        assert np.array_equal(prim, b["primary"])
+        assert reference_store.same(prim, b["primary"])
     finally:
         ref.contract_math(False)
 
@@ -327,7 +325,7 @@ def test_balance_goal_against_the_references_own_class(ref, oracle):
         prim, _ = oracle.approx_fitness(ref.effective_robot(rm), pr, ref.effective_goal_params(rm, pr, gp, B), seeds, base, genes)
     finally:
         oracle.component_flags(0)
-    assert np.array_equal(prim, b["primary"]) and np.abs(prim).min() > 0
+    assert reference_store.same(prim, b["primary"]) and np.abs(prim).min() > 0
     compare(oracle, ref, rm, pr, oracle_lib.make_cfg(population=18), gp, seeds, 1 + np.arange(B, dtype=np.uint32), 5)
     # the goal really contributes: without it the fitness differs
     rm2, groups2 = robots.balancing_tree()
